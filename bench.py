@@ -33,10 +33,10 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import time
-import uuid
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -70,7 +70,16 @@ def parse_args():
                    help="reference arm: MB written+read per step (one round)")
     p.add_argument("--quick", action="store_true",
                    help="small shapes for a functional check (256 MB x 2 rounds, no extras)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps write a fixed, seeded sample of what the last "
+                        "step read back (`dst`) to DIR/dst_sample.npy: float32, 32 MB in all "
+                        "(dst_sample_rank<r>.npy per rank with several GPUs)")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        p.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def reference_arm(args):
@@ -396,10 +405,11 @@ def main():
     offsets = [i * elems for i in range(nblocks)]
     offsets_np = np.asarray(offsets, dtype=np.int64)
     stream = torch.cuda.Stream(device=dev)
+    key_rng = random.Random(1234 + rank)  # same keys every run with the same arguments
 
     def fresh_round():
         """Keys, reserved pool blocks and the (key, offset) list of one round (untimed)."""
-        tag = uuid.uuid4().hex
+        tag = f"{key_rng.getrandbits(128):032x}"
         keys = [f"{tag}-{i:07d}" for i in range(nblocks)]
         remote = conn.allocate_rdma(keys, block_bytes)
         return remote, list(zip(keys, offsets))
@@ -478,6 +488,16 @@ def main():
                      "cpus": len(os.sched_getaffinity(0)), "numa_node": numa_node,
                      "epochs": -(-nr // pool_rounds), "rounds_per_epoch": int(pool_rounds)}
     ok = bool(torch.equal(src, dst))
+    if args.dump_outputs:
+        # one position per stride, drawn from a fixed seed: the same sample for the same arguments
+        stride = -(-dst.numel() // ((32 << 20) // 4 // world))
+        n = -(-dst.numel() // stride)
+        pos = np.arange(n) * stride + np.random.default_rng(rank).integers(0, stride, n)
+        pos = np.minimum(pos, dst.numel() - 1)
+        sample = dst.index_select(0, torch.from_numpy(pos).to(dev)).float().cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "dst_sample.npy" if world == 1 else f"dst_sample_rank{rank}.npy"
+        np.save(os.path.join(args.dump_outputs, name), sample)
 
     ms_max = allmax(ms)
     ms_per_step = ms_max / args.steps
